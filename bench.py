@@ -59,7 +59,36 @@ def parse():
                    "flags below override seq_len / micro_bsz / micro_num / sizes when given")
     p.add_argument("--pp", type=int, default=0, help="pipeline size override (with --config)")
     p.add_argument("--segments", type=int, default=1, help="equal-length packed sequences per micro-batch row")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", default=None, metavar="DIR",
+                   help="after the timed steps, write what the last one returned (loss, gradient norms, a fixed sample of "
+                        "the updated weights) as DIR/<name>.npy, to compare two builds output for output")
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
+    return a
+
+
+DUMP_PER_TENSOR = 1 << 15   # weight entries sampled per parameter: ~40 MB of float32 for the 7B model
+
+
+def dump_outputs(dst, loss, norms, model):
+    """The last timed step's results as float32 / float64 ``.npy`` files: the loss, the gradient norm of every parameter
+    group and, per parameter, the same seeded sample of entries of the updated weights (positions depend only on the
+    parameter's shape, so two runs of the same configuration sample the same entries)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(dst, exist_ok=True)
+    np.save(os.path.join(dst, "loss.npy"), np.array([float(loss)], dtype=np.float64))
+    for group, v in sorted(norms.items()):
+        np.save(os.path.join(dst, f"grad_norm.{group}.npy"), np.array([float(v)], dtype=np.float64))
+    for name, p in model.named_parameters():
+        flat = p.detach().reshape(-1)
+        if flat.numel() > DUMP_PER_TENSOR:
+            g = torch.Generator().manual_seed(flat.numel())
+            idx = torch.randint(0, flat.numel(), (DUMP_PER_TENSOR,), generator=g).sort().values
+            flat = flat[idx.to(flat.device)]
+        np.save(os.path.join(dst, f"weight.{name}.npy"), flat.float().cpu().numpy())
 
 
 def _plain(x):
@@ -335,6 +364,7 @@ def run(a, ours: bool):
     dev_batches = [({k: v.cuda() for k, v in d.items()}, l.cuda()) for d, l in host_batches]
 
     skipped = [0]   # the reference arm only reports skipped steps (its loss-scale warm-up is its own business)
+    last_norms = [None]
 
     def step_dev(batch):
         d, l = batch
@@ -342,6 +372,7 @@ def run(a, ours: bool):
         out = trainer.execute_schedule(({k: v for k, v in d.items()}, l), forward_only=False, return_loss=True,
                                        return_output_label=False)
         ok, norms = trainer.step()
+        last_norms[0] = norms
         if not ok:  # overflow / non-finite gradients: the optimizer skipped its update -> not the benchmark's work
             skipped[0] += 1
             if ours:
@@ -367,6 +398,8 @@ def run(a, ours: bool):
     e2e_ms, e2e_wall, _, last_e2e = timed_loop(torch, dist, step_e2e, host_batches, a.steps, world, None, finish,
                                                first=a.warmup + a.steps + 1)
     e2e_ms = max(e2e_ms, e2e_wall)  # the host read-back is part of the region: take the host clock if it is longer
+    if a.dump_outputs and rank == 0 and last_e2e is not None:
+        dump_outputs(a.dump_outputs, last_e2e, last_norms[0], model)
 
     tokens_per_step = T * a.micro_num * dp
     value = tokens_per_step * a.steps / (ms / 1e3)
@@ -449,7 +482,7 @@ def _tp2_args(a):
     import copy
 
     b = copy.copy(a)
-    b.tp, b.tp_mode, b.no_tp2 = 2, "mtp", True
+    b.tp, b.tp_mode, b.no_tp2, b.dump_outputs = 2, "mtp", True, None
     return b
 
 

@@ -13,6 +13,40 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 
+GOLDEN = os.path.join(ROOT, "tests", "golden", "reference")
+REFERENCE = os.environ.get("INTERNEVO_REFERENCE")
+
+
+def reference_output(name, make):
+    """Path of what the reference computed for ``name``, stored under ``tests/golden/reference``.  With ``INTERNEVO_REFERENCE``
+    set to a checkout of the reference, ``make(reference_root, path)`` runs the reference and stores its result there first."""
+    path = os.path.join(GOLDEN, name)
+    if REFERENCE:
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        make(REFERENCE, path)
+    assert os.path.exists(path), path
+    return path
+
+
+def assert_close(a, b, where):
+    """``a`` equals ``b`` key by key, tensors to float rounding (computed on another CPU, in another order)."""
+    if isinstance(a, dict):
+        assert isinstance(b, dict) and sorted(a, key=str) == sorted(b, key=str), (where, sorted(a, key=str), sorted(b, key=str))
+        for k in a:
+            assert_close(a[k], b[k], f"{where}/{k}")
+    elif isinstance(a, (list, tuple)):
+        assert isinstance(b, (list, tuple)) and len(a) == len(b), where
+        for i, (x, y) in enumerate(zip(a, b)):
+            assert_close(x, y, f"{where}/{i}")
+    elif isinstance(a, torch.Tensor):
+        assert a.shape == b.shape and a.dtype == b.dtype, (where, a.shape, b.shape, a.dtype, b.dtype)
+        assert torch.allclose(a.double(), b.double(), rtol=1e-4, atol=1e-6), (where, float((a.double() - b.double()).abs().max()))
+    elif isinstance(a, float):
+        assert abs(a - b) <= 1e-6 * max(1.0, abs(a)), (where, a, b)
+    else:
+        assert a == b, (where, a, b)
+
+
 def find_free_port():
     with socket.socket(socket.AF_INET, socket.SOCK_STREAM) as s:
         s.bind(("127.0.0.1", 0))

@@ -1,11 +1,16 @@
 import os
 import sys
+import tempfile
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+
+# the remote code of converted checkpoints that transformers caches (``trust_remote_code``) goes to a temporary directory, not
+# to a home directory that may not be writable; set here, before any test imports transformers, so that sub-processes inherit it
+os.environ["HF_HOME"] = os.path.join(tempfile.gettempdir(), f"internevo-tests-hf-{os.getuid()}")
 
 
 def pytest_configure(config):

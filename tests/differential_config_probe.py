@@ -1,7 +1,8 @@
 """``args_sanity_check`` on one of the reference's OWN config files, run against the reference and against this repository
-(``internlm`` alias); prints the resulting configuration (see ``test_reference_differential_cpu.py``).
+(``internlm`` alias); prints the resulting configuration (see ``test_reference_differential_cpu.py``).  A ``.json`` config holds
+the values a config file defines, as ``Config.from_file`` loaded them.
 
-    python differential_config_probe.py <root that provides `internlm`> <config file> <output json>
+    python differential_config_probe.py <root that provides `internlm`> <config file or .json> <output json>
 """
 import json
 import sys
@@ -13,7 +14,7 @@ from internlm.core.context import ParallelMode  # noqa: E402
 from internlm.core.context import global_context as gpc  # noqa: E402
 from internlm.core.context.parallel_context import Config  # noqa: E402
 
-gpc._config = Config.from_file(cfgfile)
+gpc._config = Config(json.load(open(cfgfile))) if cfgfile.endswith(".json") else Config.from_file(cfgfile)
 gpc.is_rank_for_log = lambda: False
 gpc.get_world_size = lambda mode: 8 if mode in (ParallelMode.GLOBAL, ParallelMode.DATA) else 1   # an 8-GPU data-parallel job
 gpc.is_initialized = lambda mode: True

@@ -38,7 +38,7 @@ if which == "load":        # the converted model's MLP width (the trainer rounds
     shapes = {k: v.shape for k, v in torch.load(prefix + ".hf_weights").items()}
     kw["intermediate_size"] = next(v[0] for k, v in shapes.items() if k.endswith("feed_forward.w1.weight") or k.endswith("gate_proj.weight"))
 cfg = getattr(cfg_mod, name + "Config")(**kw)
-if which in ("ref", "load") and base.startswith("/root/reference") and getattr(cfg, "rope_scaling", None) is not None:
+if which in ("ref", "load") and getattr(cfg, "rope_scaling", None) is not None:     # "ref" / "load" run the reference's code
     cfg.rope_scaling = None       # transformers 5 fills in a rope dict the 4.x-era reference code does not understand
 if which == "ref" and family == "internlm" and hasattr(cfg, "rotary"):
     pass

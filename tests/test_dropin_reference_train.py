@@ -1,16 +1,16 @@
-"""Drop-in check: the REFERENCE's own, unmodified `train.py` (taken from the read-only reference checkout at test time into
-pytest's temp dir, so that the script's directory does not put the reference package first on `sys.path`; nothing of it
-lives in this repo) runs against this framework — its `import internlm...` lines resolve to `internevo_b200` through the alias package
-— and trains the demo config on 2 CPU ranks to the same final loss as our `train.py`."""
+"""Drop-in check: the REFERENCE's own, unmodified `train.py` runs against this framework - its `import internlm...` lines resolve to
+`internevo_b200` through the alias package - and trains the demo config on 2 CPU ranks to the same losses as our `train.py`.  The
+losses of the reference's script are stored under `tests/golden/reference` (nothing of the script lives in this repo);
+`INTERNEVO_REFERENCE=<checkout of the reference>` runs it again (from pytest's temp dir, so that the script's directory does not
+put the reference package first on `sys.path`) and rewrites them."""
+import json
 import os
 import re
 import subprocess
 import sys
 
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_TRAIN = "/root/reference/train.py"
 
 
 def _losses(script, port, cwd):
@@ -22,16 +22,18 @@ def _losses(script, port, cwd):
     return [float(x) for x in re.findall(r"step=\d+ loss=([0-9.]+)", r.stdout + r.stderr)]
 
 
-@pytest.mark.skipif(not os.path.exists(REF_TRAIN), reason="reference checkout not present")
 def test_reference_train_py_runs_on_this_framework(tmp_path):
     sys.path.insert(0, os.path.join(ROOT, "tests"))
-    from common import find_free_port
+    from common import find_free_port, reference_output
 
     import shutil
 
-    script = str(tmp_path / "reference_train.py")
-    shutil.copy(REF_TRAIN, script)
-    theirs = _losses(script, find_free_port(), str(tmp_path))
+    def make(root, dst):
+        script = str(tmp_path / "reference_train.py")
+        shutil.copy(os.path.join(root, "train.py"), script)
+        json.dump(_losses(script, find_free_port(), str(tmp_path)), open(dst, "w"))
+
+    theirs = json.load(open(reference_output("dropin_train_losses.json", make)))
     ours = _losses(os.path.join(ROOT, "train.py"), find_free_port(), str(tmp_path))
     assert len(theirs) == len(ours) == 20
     assert theirs[-1] < 1.5 < theirs[0]

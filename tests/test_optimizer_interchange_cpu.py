@@ -115,16 +115,14 @@ def test_reference_format_round_trip_is_exact(tmp_path):
 
 
 def test_partition_matches_the_reference_implementation():
-    """``reference_partition`` against the reference's own ``_partition_param_list`` (run unbound on a stub) when the reference
-    is installed under ``baseline/_ref``."""
-    ref = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
-    if not os.path.isdir(os.path.join(ref, "internlm")):
-        pytest.skip("baseline/_ref is not installed")
+    """``reference_partition`` against the plans of the reference's own ``_partition_param_list`` (run unbound on a stub)."""
     import subprocess
+
+    from common import reference_output
 
     code = f'''
 import sys, types, json, torch
-sys.path.insert(0, {ref!r})
+sys.path.insert(0, sys.argv.pop(1))
 from internlm.solver.optimizer.hybrid_zero_optim import HybridZeroOptimizer
 from internlm.core.context import global_context as gpc
 gpc.is_rank_for_log = lambda: False
@@ -139,11 +137,19 @@ print("PLAN" + json.dumps(stub.params_per_rank_id_dict[0]))
     from internevo_b200.checkpoint.optimizer_interchange import reference_partition
 
     shapes = [[128, 64], [64], [192, 64], [64, 64], [64], [64], [256, 64], [64, 256], [256, 64], [64], [128, 64], [7, 3]]
+
+    def make(ref, dst):
+        plans = {}
+        for world in (1, 2, 3, 4):
+            r = subprocess.run([sys.executable, "-c", code, ref, json.dumps(shapes), str(world)], capture_output=True, text=True,
+                               timeout=300, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+            assert r.returncode == 0, r.stderr[-2000:]
+            plans[world] = json.loads([line for line in r.stdout.splitlines() if line.startswith("PLAN")][0][4:])
+        json.dump(plans, open(dst, "w"))
+
+    plans = json.load(open(reference_output("partition_plans.json", make)))
     for world in (1, 2, 3, 4):
-        r = subprocess.run([sys.executable, "-c", code, json.dumps(shapes), str(world)], capture_output=True, text=True,
-                           timeout=300, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-        assert r.returncode == 0, r.stderr[-2000:]
-        theirs = json.loads([line for line in r.stdout.splitlines() if line.startswith("PLAN")][0][4:])
+        theirs = plans[str(world)]
         _, ours = reference_partition(shapes, world)
         assert ours == theirs, (world, ours, theirs)
 
@@ -219,18 +225,29 @@ def test_the_references_own_loader_accepts_the_exported_files(tmp_path):
     (run unbound on a stub that carries what its ``__init__`` would have built: the parameter partition from its own
     ``_partition_param_list``, one flat fp32 buffer + ``torch.optim.AdamW`` per rank).  torch validates the AdamW state dict, the
     reference its buffer shapes, and afterwards its master buffer equals the weights of its model file parameter by parameter -
-    which pins the parameter order and the ``w13`` → ``w1`` / ``w3`` translation."""
+    which pins the parameter order and the ``w13`` → ``w1`` / ``w3`` translation.  The files the reference accepted are stored;
+    the files exported here must equal them."""
     import json
+    import shutil
     import subprocess
 
+    from common import assert_close, reference_output
     from internevo_b200.checkpoint.optimizer_interchange import _reference_order
 
-    ref = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
-    if not os.path.isdir(os.path.join(ref, "internlm")):
-        pytest.skip("baseline/_ref is not installed")
     run_distributed(_run, 2, str(tmp_path), "first", 2, "reference")
     folder = os.path.join(str(tmp_path), "2")
-    keys = _reference_order(list(torch.load(os.path.join(folder, "model_tp0_pp0.pt"), weights_only=False).keys()))
-    r = subprocess.run([sys.executable, "-c", _REFERENCE_LOADER, ref, folder, "2", json.dumps(keys)], capture_output=True,
-                       text=True, timeout=600, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-    assert r.returncode == 0 and "REFERENCE_LOADED_OK" in r.stdout, r.stderr[-3000:]
+    files = ("model_tp0_pp0.pt", "optimizer_tp0_pp0_zo0.pt", "optimizer_tp0_pp0_zo1.pt")
+
+    def make(ref, dst):
+        keys = _reference_order(list(torch.load(os.path.join(folder, "model_tp0_pp0.pt"), weights_only=False).keys()))
+        r = subprocess.run([sys.executable, "-c", _REFERENCE_LOADER, ref, folder, "2", json.dumps(keys)], capture_output=True,
+                           text=True, timeout=600, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+        assert r.returncode == 0 and "REFERENCE_LOADED_OK" in r.stdout, r.stderr[-3000:]
+        os.makedirs(dst, exist_ok=True)
+        for fn in files:
+            shutil.copy(os.path.join(folder, fn), dst)
+
+    accepted = reference_output("optimizer_files_accepted", make)
+    for fn in files:
+        assert_close(torch.load(os.path.join(folder, fn), weights_only=False),
+                     torch.load(os.path.join(accepted, fn), weights_only=False), fn)

@@ -2,6 +2,7 @@
 behave (reference paths cited next to each implementation)."""
 import ast
 import importlib
+import json
 import math
 import os
 import sys
@@ -9,34 +10,39 @@ import sys
 import pytest
 import torch
 
-from common import ROOT, run_distributed  # noqa: F401
+from common import ROOT, reference_output, run_distributed  # noqa: F401
 
-REF = "/root/reference/internlm"
 # by design: one accelerator backend
 NO_COUNTERPART = {"internlm.accelerator.npu_accelerator"}
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
-def test_every_reference_module_path_resolves():
-    missing, names, absent = [], 0, 0
-    for d, _, fs in sorted(os.walk(REF)):
+def _reference_modules(root, dst):
+    """Every module of the reference's ``internlm`` package with the public classes / functions it defines."""
+    tree, out = os.path.join(root, "internlm"), {}
+    for d, _, fs in sorted(os.walk(tree)):
         for f in sorted(fs):
-            if not f.endswith(".py"):
-                continue
-            path = os.path.join(d, f)
-            mod = os.path.relpath(path, os.path.dirname(REF))[:-3].replace("/", ".")
-            mod = mod[:-9] if mod.endswith(".__init__") else mod
-            if mod in NO_COUNTERPART:
-                continue
-            try:
-                m = importlib.import_module(mod)
-            except Exception as e:  # noqa: BLE001
-                missing.append((mod, repr(e)[:80]))
-                continue
-            for node in ast.parse(open(path).read()).body:
-                if isinstance(node, (ast.ClassDef, ast.FunctionDef)) and not node.name.startswith("_"):
-                    names += 1
-                    absent += not hasattr(m, node.name)
+            if f.endswith(".py"):
+                path = os.path.join(d, f)
+                mod = os.path.relpath(path, root)[:-3].replace(os.sep, ".")
+                mod = mod[:-9] if mod.endswith(".__init__") else mod
+                out[mod] = [node.name for node in ast.parse(open(path).read()).body
+                            if isinstance(node, (ast.ClassDef, ast.FunctionDef)) and not node.name.startswith("_")]
+    json.dump(out, open(dst, "w"), indent=0)
+
+
+def test_every_reference_module_path_resolves():
+    modules = json.load(open(reference_output("modules.json", _reference_modules)))
+    missing, names, absent = [], 0, 0
+    for mod, public in modules.items():
+        if mod in NO_COUNTERPART:
+            continue
+        try:
+            m = importlib.import_module(mod)
+        except Exception as e:  # noqa: BLE001
+            missing.append((mod, repr(e)[:80]))
+            continue
+        names += len(public)
+        absent += sum(not hasattr(m, name) for name in public)
     assert not missing, missing
     # every public class / function of the reference is reachable under its own name
     assert names > 300 and absent == 0, (names, absent)

@@ -1,34 +1,35 @@
 """Differential tests against the UNMODIFIED reference: ``tests/differential_probe.py`` - written only against the reference's import
-paths and signatures - runs once with the reference first on ``sys.path`` (``baseline/_ref`` or ``/root/reference``) and once with
-this repository, whose ``internlm`` package is an alias of ``internevo_b200``.  Everything a loss curve depends on outside the
+paths and signatures - runs with this repository, whose ``internlm`` package is an alias of ``internevo_b200``, and its results are
+compared with what the same probe computed with the reference first on ``sys.path``.  The reference's results are stored under
+``tests/golden/reference``; ``INTERNEVO_REFERENCE=<checkout of the reference> pytest tests/test_reference_differential_cpu.py``
+computes them afresh from the reference and rewrites them.  Everything a loss curve depends on outside the
 kernels is compared value by value: sampler batches (ramp-up, epoch roll-over, resume), tokenized-file reading, both packed
 datasets item by item, collate functions, learning-rate / beta2 schedules, the dynamic loss scaler, the reported TFLOPS and the
 layer partition."""
 import json
 import math
 import os
+import shutil
 import subprocess
 import sys
 
 import numpy as np
 import pytest
 
+from common import assert_close, reference_output
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PROBE = os.path.join(ROOT, "tests", "differential_probe.py")
 
 
-def _reference_root():
-    for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(os.path.join(cand, "internlm", "data", "tokenized")):
-            return cand
-    return None
+def _probe(script, *args, cwd, timeout=600, **env):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", script), *map(str, args)], capture_output=True, text=True,
+                       timeout=timeout, cwd=str(cwd), env=dict(os.environ, CUDA_VISIBLE_DEVICES="", **env))
+    assert r.returncode == 0 and "PROBE_OK" in r.stdout, f"{script} {args}: {r.stderr[-3000:]}"
 
 
 @pytest.fixture(scope="module")
 def both(tmp_path_factory):
-    ref = _reference_root()
-    if ref is None:
-        pytest.skip("the reference is not installed (baseline/_ref)")
     import sentencepiece as spm
 
     work = tmp_path_factory.mktemp("differential")
@@ -42,14 +43,9 @@ def both(tmp_path_factory):
     subprocess.run([sys.executable, os.path.join(ROOT, "tools", "tokenizer.py"), "--text_input_path", str(corpus),
                     "--bin_output_path", str(work / "en" / "part0.bin"), "--tokenizer_model", str(work / "tok.model")],
                    check=True, capture_output=True)
-    res = {}
-    for side, root in (("reference", ref), ("ours", ROOT)):
-        dst = str(work / f"{side}.json")
-        r = subprocess.run([sys.executable, PROBE, root, str(work), dst], capture_output=True, text=True, timeout=600,
-                           cwd=str(work), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-        assert r.returncode == 0 and "PROBE_OK" in r.stdout, f"{side}: {r.stderr[-3000:]}"
-        res[side] = json.load(open(dst))
-    return res["reference"], res["ours"]
+    ref = reference_output("probe.json", lambda root, dst: _probe(PROBE, root, work, dst, cwd=work))
+    _probe(PROBE, ROOT, work, work / "ours.json", cwd=work)
+    return json.load(open(ref)), json.load(open(work / "ours.json"))
 
 
 def _same(a, b, tol=0.0):
@@ -107,18 +103,21 @@ def test_args_sanity_check_fills_a_reference_config_like_the_reference(tmp_path,
     """A config file SHIPPED BY THE REFERENCE goes through ``args_sanity_check`` on both sides: every default it fills in, every
     derived key (``sequence_parallel``, ``packed_length``, checkpoint sub-keys, monitor section, MoE / ISP switches ...) comes
     out identical - the configuration a reference user brings along means the same thing here."""
-    ref = _reference_root()
-    src = next((p for p in (os.path.join("/root/reference/configs", config + ".py"),
-                            os.path.join(ref or "", "..", "..", "configs", config + ".py")) if os.path.exists(p)), None)
-    if ref is None or src is None:
-        pytest.skip("the reference (and its configs folder) is not available")
+    def make_input(root, dst):
+        code = ("import json, sys; sys.path.insert(0, sys.argv[1]); from internlm.core.context.parallel_context import Config; "
+                "json.dump(dict(Config.from_file(sys.argv[2])), open(sys.argv[3], 'w'), indent=1, sort_keys=True)")
+        subprocess.run([sys.executable, "-c", code, root, os.path.join(root, "configs", config + ".py"), dst], check=True,
+                       cwd=str(tmp_path), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+
+    src = reference_output(f"config_{config}.json", make_input)
     out = {}
-    for side, root in (("reference", ref), ("ours", ROOT)):
+    for side, root in (("reference", None), ("ours", ROOT)):
         dst = str(tmp_path / f"{side}.json")
-        r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_config_probe.py"), root, src, dst],
-                           capture_output=True, text=True, timeout=600, cwd=str(tmp_path),
-                           env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-        assert r.returncode == 0 and "PROBE_OK" in r.stdout, f"{side}: {r.stderr[-3000:]}"
+        if root is None:
+            dst = reference_output(f"config_{config}.checked.json",
+                                   lambda root, dst: _probe("differential_config_probe.py", root, src, dst, cwd=tmp_path))
+        else:
+            _probe("differential_config_probe.py", root, src, dst, cwd=tmp_path)
         out[side] = json.load(open(dst))
 
     def flat(d, prefix=""):
@@ -162,6 +161,10 @@ def test_top1_gating_without_random_token_selection(both, key):
     assert kept[0] == kept[1] == [min(c, torch.tensor(ref[key]["combine"]).shape[2]) for c in ref[key]["counts"]]
 
 
+def _model_probe(family, cwd):
+    return reference_output(f"model_{family}.pt", lambda root, dst: _probe("differential_model_probe.py", root, family, dst, cwd=cwd))
+
+
 def _our_logits(rank, world, family, ref_file):
     import torch
 
@@ -202,13 +205,7 @@ def test_model_forward_equals_the_references_on_its_own_weights(tmp_path, family
     equal RNG state above)."""
     from common import run_distributed
 
-    ref = _reference_root()
-    if ref is None:
-        pytest.skip("the reference is not installed (baseline/_ref)")
-    dst = str(tmp_path / f"{family}.pt")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_model_probe.py"), ref, family, dst],
-                       capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-    assert r.returncode == 0 and "PROBE_OK" in r.stdout, r.stderr[-3000:]
+    dst = _model_probe(family, tmp_path)
     ours, theirs, moe, their_moe = run_distributed(_our_logits, 1, family, dst)[0]
     assert ours.shape == theirs.shape
     assert float((ours - theirs).abs().max()) < 2e-6 * max(1.0, float(theirs.abs().max())), float((ours - theirs).abs().max())
@@ -226,6 +223,7 @@ def _our_training(rank, world, ref_file, family="INTERNLM2_PUBLIC"):
     from internevo_b200.train import get_scheduler_hooks, initialize_model, initialize_optimizer
 
     ref = torch.load(ref_file, weights_only=False)
+    ref["final"] = torch.load(ref_file[:-3] + ".final.pt", weights_only=False)
     S, MB, MN = 16, 2, 2
     cfg = tiny_config(model_type=family, num_layers=2, hidden=32, heads=4, kv_heads=2, vocab=64, seq_len=S, micro_bsz=MB,
                       micro_num=MN)
@@ -278,15 +276,18 @@ def test_eight_training_steps_follow_the_reference(tmp_path, family):
     position among NON-EMPTY groups (``hybrid_zero_optim.py:863-876``), i.e. it takes the factor of the empty ``default`` group
     and never clips, while bf16 runs (groups aligned) clip like this framework; (2) the schedule is long, so the factor
     ``2 / (1 + cos(pi / T))`` that torch's recursive cosine puts on the reference's learning rate is below 1e-5."""
+    import torch
+
     from common import run_distributed
 
-    ref = _reference_root()
-    if ref is None:
-        pytest.skip("the reference is not installed (baseline/_ref)")
-    dst = str(tmp_path / "train.pt")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_train_probe.py"), ref, dst, family],
-                       capture_output=True, text=True, timeout=900, cwd=str(tmp_path), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-    assert r.returncode == 0 and "PROBE_OK" in r.stdout, r.stderr[-3000:]
+    def make(root, dst):
+        # the final weights in a file of their own: no stored file is larger than 1 MB
+        _probe("differential_train_probe.py", root, dst, family, cwd=tmp_path, timeout=900)
+        ref = torch.load(dst, weights_only=False)
+        torch.save(ref.pop("final"), dst[:-3] + ".final.pt")
+        torch.save(ref, dst)
+
+    dst = reference_output(f"train_{family}.pt", make)
     losses, ref_losses, norms, ref_norms, drift, moved = run_distributed(_our_training, 1, dst, family)[0]
     assert len(losses) == len(ref_losses) == 8
     for a, b in zip(losses, ref_losses):
@@ -364,13 +365,17 @@ def test_a_checkpoint_written_by_the_reference_resumes_here(tmp_path):
     learning-rate schedule all arrive through the files (``checkpoint/optimizer_interchange.py``)."""
     from common import run_distributed
 
-    ref = _reference_root()
-    if ref is None:
-        pytest.skip("the reference is not installed (baseline/_ref)")
-    dst, folder = str(tmp_path / "train.pt"), str(tmp_path / "ref_ckpt")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_train_probe.py"), ref, dst, "INTERNLM2_PUBLIC", folder],
-                       capture_output=True, text=True, timeout=900, cwd=str(tmp_path), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-    assert r.returncode == 0 and "PROBE_OK" in r.stdout, r.stderr[-3000:]
+    def make(root, dst):
+        shutil.rmtree(dst, ignore_errors=True)
+        os.makedirs(dst)
+        _probe("differential_train_probe.py", root, os.path.join(dst, "train.pt"), "INTERNLM2_PUBLIC", os.path.join(dst, "ckpt"),
+               cwd=tmp_path, timeout=900)
+        for fn in os.listdir(os.path.join(dst, "ckpt")):      # only the checkpoint after step 4 is resumed
+            if fn not in ("4", "4.step"):
+                shutil.rmtree(os.path.join(dst, "ckpt", fn), ignore_errors=True)
+
+    base = reference_output("checkpoint_from_reference", make)
+    dst, folder = os.path.join(base, "train.pt"), os.path.join(base, "ckpt")
     assert {"model_tp0_pp0.pt", "optimizer_tp0_pp0_zo0.pt", "schedulder.pt", "context.pt", "4.step"} <= set(os.listdir(f"{folder}/4"))
     losses, ref_losses, drift, moved = run_distributed(_resume_reference_checkpoint, 1, dst, folder)[0]
     assert len(losses) == 4
@@ -440,16 +445,21 @@ def test_the_reference_resumes_a_checkpoint_written_here(tmp_path):
 
     from common import run_distributed
 
-    ref = _reference_root()
-    if ref is None:
-        pytest.skip("the reference is not installed (baseline/_ref)")
-    folder, dst = str(tmp_path / "our_ckpt"), str(tmp_path / "resumed.pt")
+    folder = str(tmp_path / "our_ckpt")
     losses, final = run_distributed(_train_and_save_for_the_reference, 1, folder)[0]
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_train_probe.py"), ref, dst, "INTERNLM2_PUBLIC", folder,
-                        "resume"], capture_output=True, text=True, timeout=900, cwd=str(tmp_path),
-                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-    assert r.returncode == 0 and "PROBE_OK" in r.stdout, r.stderr[-3000:]
-    theirs = torch.load(dst, weights_only=False)
+
+    def make(root, dst):
+        shutil.rmtree(dst, ignore_errors=True)
+        shutil.copytree(os.path.join(folder, "4"), os.path.join(dst, "loaded", "4"))
+        _probe("differential_train_probe.py", root, os.path.join(dst, "resumed.pt"), "INTERNLM2_PUBLIC", os.path.join(dst, "loaded"),
+               "resume", cwd=tmp_path, timeout=900)
+
+    base = reference_output("checkpoint_for_reference", make)
+    # the files written here are the ones the reference was shown to load
+    for fn in ("model_tp0_pp0.pt", "optimizer_tp0_pp0_zo0.pt", "schedulder.pt"):
+        assert_close(torch.load(os.path.join(folder, "4", fn), weights_only=False),
+                      torch.load(os.path.join(base, "loaded", "4", fn), weights_only=False), fn)
+    theirs = torch.load(os.path.join(base, "resumed.pt"), weights_only=False)
     assert len(theirs["losses"]) == 4
     for a, b in zip(theirs["losses"], losses[4:]):
         assert abs(a - b) < 2e-6 * max(1.0, abs(b)), (theirs["losses"], losses[4:])
@@ -485,17 +495,13 @@ def test_train_and_validation_loaders_yield_the_references_batches(data_folder, 
     sample filtering (``min_length`` for training, 50 tokens for validation), packing, the sampler's order and the collated batch -
     the first six training batches and the first two batches of every validation set are identical, tensor by tensor, on both
     data-parallel ranks and in both packing modes."""
-    ref = _reference_root()
-    if ref is None:
-        pytest.skip("the reference is not installed (baseline/_ref)")
-    out = {}
-    for side, root in (("reference", ref), ("ours", ROOT)):
-        dst = str(data_folder / f"{side}_{dp_rank}_{pack}.json")
-        r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_loader_probe.py"), root,
-                            str(data_folder / "data"), dst] + (["one"] if pack == "one" else []), capture_output=True, text=True,
-                           timeout=600, cwd=str(data_folder), env=dict(os.environ, CUDA_VISIBLE_DEVICES="", PROBE_DP_RANK=str(dp_rank)))
-        assert r.returncode == 0 and "PROBE_OK" in r.stdout, f"{side}: {r.stderr[-3000:]}"
-        out[side] = json.load(open(dst))
+    def run(root, dst):
+        _probe("differential_loader_probe.py", root, data_folder / "data", dst, *(["one"] if pack == "one" else []), cwd=data_folder,
+               PROBE_DP_RANK=str(dp_rank))
+
+    dst = str(data_folder / f"ours_{dp_rank}_{pack}.json")
+    run(ROOT, dst)
+    out = {"ours": json.load(open(dst)), "reference": json.load(open(reference_output(f"loader_{dp_rank}_{pack}.json", run)))}
     a, b = out["reference"], out["ours"]
     assert a["types"] == b["types"] == ["cn", "code", "en"] and a["len"] == b["len"] > 6
     for i, (x, y) in enumerate(zip(a["batches"], b["batches"])):
@@ -507,16 +513,11 @@ def test_metrics_report_the_references_keys_and_values(tmp_path):
     """Accuracy, perplexity, ``loss_from_metric`` and the per-type ``acc/`` ``tokens/`` ``loss/`` entries of the step log: every key
     the reference's ``AccPerplex`` / ``LossWithTypeId`` return is returned here with the same value (this framework adds
     ``perplexity/<type>``)."""
-    ref = _reference_root()
-    if ref is None:
-        pytest.skip("the reference is not installed (baseline/_ref)")
-    out = {}
-    for side, root in (("reference", ref), ("ours", ROOT)):
-        dst = str(tmp_path / f"{side}.json")
-        r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_metric_probe.py"), root, dst], capture_output=True,
-                           text=True, timeout=600, cwd=str(tmp_path), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-        assert r.returncode == 0 and "PROBE_OK" in r.stdout, f"{side}: {r.stderr[-3000:]}"
-        out[side] = json.load(open(dst))
+    def run(root, dst):
+        _probe("differential_metric_probe.py", root, dst, cwd=tmp_path)
+
+    run(ROOT, tmp_path / "ours.json")
+    out = {"ours": json.load(open(tmp_path / "ours.json")), "reference": json.load(open(reference_output("metrics.json", run)))}
     for part in ("acc", "loss"):
         theirs, ours = out["reference"][part], out["ours"][part]
         assert set(theirs) <= set(ours), (part, sorted(set(theirs) - set(ours)))
@@ -524,26 +525,51 @@ def test_metrics_report_the_references_keys_and_values(tmp_path):
             assert abs(v - ours[k]) < 1e-4 * max(1.0, abs(v)), (k, v, ours[k])
 
 
+def _small_tokenizer_model(cwd):
+    """A small SentencePiece model (the reference's own is 1.6 MB) on which both code bases' tokenizer tools run."""
+    def make(root, dst):
+        import sentencepiece as spm
+
+        rng = np.random.RandomState(11)
+        words = ["alpha", "beta", "gamma", "delta", "epsilon", "zeta", "eta", "theta", "iota", "kappa", "训练", "模型", "数据"]
+        (cwd / "spm.txt").write_text("\n".join(" ".join(rng.choice(words, rng.randint(1, 30))) for _ in range(400)))
+        spm.SentencePieceTrainer.Train(input=str(cwd / "spm.txt"), model_prefix=str(cwd / "spm"), vocab_size=96, bos_id=1,
+                                       eos_id=2, unk_id=0, pad_id=-1, model_type="bpe", character_coverage=1.0,
+                                       normalization_rule_name="identity", minloglevel=2)
+        shutil.copy(cwd / "spm.model", dst)
+
+    return reference_output("tokenizer_small.model", make)
+
+
 def test_tokenizer_tool_writes_the_references_bytes(tmp_path):
-    """``tools/tokenizer.py`` of both code bases on the same text with the reference's own SentencePiece model: the ``.bin`` files
-    are byte-identical and the ``.meta`` offsets / lengths equal (kept int64 here - the reference's int32 wraps beyond 2 GiB)."""
-    ref_tool, model = "/root/reference/tools/tokenizer.py", "/root/reference/tools/tokenizer_internlm.model"
-    if not (os.path.exists(ref_tool) and os.path.exists(model)):
-        pytest.skip("the reference's tools folder is not available")
+    """``tools/tokenizer.py`` of both code bases on the same text with the same SentencePiece model: the ``.bin`` files are
+    byte-identical and the ``.meta`` offsets / lengths equal (kept int64 here - the reference's int32 wraps beyond 2 GiB)."""
+    model = _small_tokenizer_model(tmp_path)
     rng = np.random.RandomState(5)
     words = ["alpha", "beta", "gamma", "delta", "epsilon", "zeta", "eta", "theta", "iota", "kappa", "训练", "模型", "数据"]
     text = tmp_path / "corpus.txt"
     text.write_text("\n".join(" ".join(rng.choice(words, rng.randint(1, 40))) for _ in range(200)))
     env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
-    r = subprocess.run([sys.executable, ref_tool, "--text_input_path", str(text), "--bin_output_path", str(tmp_path / "ref.bin")],
-                       capture_output=True, text=True, timeout=600, cwd="/root/reference", env=env)
-    assert r.returncode == 0, r.stderr[-2000:]
+
+    def make(root, dst):
+        # the reference's tool reads the model next to itself and its tokenizer class from ../transformers
+        os.makedirs(tmp_path / "ref" / "tools")
+        shutil.copy(os.path.join(root, "tools", "tokenizer.py"), tmp_path / "ref" / "tools")
+        shutil.copy(model, tmp_path / "ref" / "tools" / "tokenizer_internlm.model")
+        os.symlink(os.path.join(root, "transformers"), tmp_path / "ref" / "transformers")
+        r = subprocess.run([sys.executable, str(tmp_path / "ref" / "tools" / "tokenizer.py"), "--text_input_path", str(text),
+                            "--bin_output_path", dst + ".bin"], capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=env)
+        assert r.returncode == 0, r.stderr[-2000:]
+        os.replace(dst + ".bin", dst)
+
+    ref = reference_output("tokenizer.bin", make)
+    ref_meta = reference_output("tokenizer.bin.meta", lambda root, dst: os.replace(ref + ".bin.meta", dst))
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "tokenizer.py"), "--text_input_path", str(text),
                         "--bin_output_path", str(tmp_path / "ours.bin"), "--tokenizer_model", model], capture_output=True, text=True,
                        timeout=600, cwd=str(tmp_path), env=env)
     assert r.returncode == 0, r.stderr[-2000:]
-    assert open(tmp_path / "ref.bin", "rb").read() == open(tmp_path / "ours.bin", "rb").read()
-    a, b = np.load(tmp_path / "ref.bin.meta", allow_pickle=True), np.load(tmp_path / "ours.bin.meta", allow_pickle=True)
+    assert open(ref, "rb").read() == open(tmp_path / "ours.bin", "rb").read()
+    a, b = np.load(ref_meta, allow_pickle=True), np.load(tmp_path / "ours.bin.meta", allow_pickle=True)
     assert a.shape == b.shape and (a == b).all()
 
 
@@ -591,13 +617,8 @@ def test_validation_reports_the_references_numbers(data_folder, tmp_path):
     validation sets with the same number of batches, and per set the same ``val/<name>_loss`` / ``_acc`` / ``_plex`` scalars."""
     from common import run_distributed
 
-    ref = _reference_root()
-    if ref is None:
-        pytest.skip("the reference is not installed (baseline/_ref)")
-    dst = str(tmp_path / "eval.pt")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_eval_probe.py"), ref, dst, str(data_folder / "data")],
-                       capture_output=True, text=True, timeout=900, cwd=str(tmp_path), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-    assert r.returncode == 0 and "PROBE_OK" in r.stdout, r.stderr[-3000:]
+    dst = reference_output("eval.pt", lambda root, dst: _probe("differential_eval_probe.py", root, dst, data_folder / "data",
+                                                               cwd=tmp_path, timeout=900))
     ours, sizes, theirs, their_sizes = run_distributed(_our_evaluation, 1, dst, str(data_folder / "data"))[0]
     assert sizes == their_sizes and sorted(sizes) == ["cn", "code", "en"]
     keys = {k for k in theirs if k != "step"}
@@ -615,10 +636,14 @@ def test_hf_remote_code_equals_the_references(tmp_path, family):
     loads it without a missing or unexpected key and computes the same logits."""
     import torch
 
-    theirs = f"/root/reference/transformers/{family}_model"
-    if not os.path.isdir(theirs):
-        pytest.skip("the reference's transformers folder is not available")
+    def make(root, dst):
+        os.makedirs(dst, exist_ok=True)
+        _probe("differential_hf_probe.py", "ref", os.path.join(root, "transformers", f"{family}_model"), family,
+               os.path.join(dst, "m"), cwd=tmp_path)
+
+    theirs = reference_output(f"hf_{family}", make)
     prefix = str(tmp_path / family)
+    shutil.copy(os.path.join(theirs, "m.weights"), prefix + ".weights")
     # ours the way ``tools/convert2hf.py::install_remote_code`` puts it next to converted weights: one flat folder (the v1 files
     # import the shared helpers from the InternLM2 files)
     flat = tmp_path / "remote_code"
@@ -628,11 +653,8 @@ def test_hf_remote_code_equals_the_references(tmp_path, family):
             if fn.endswith(".py") and fn != "__init__.py":
                 src = open(os.path.join(ROOT, "huggingface", sub, fn)).read().replace("from ..internlm2_model.", "from .")
                 (flat / fn).write_text(src)
-    for which, base in (("ref", theirs), ("ours", str(flat))):
-        r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_hf_probe.py"), which, base, family, prefix],
-                           capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-        assert r.returncode == 0 and "PROBE_OK" in r.stdout, f"{which}: {r.stderr[-3000:]}"
-    a, b = torch.load(prefix + ".ref.logits"), torch.load(prefix + ".ours.logits")
+    _probe("differential_hf_probe.py", "ours", flat, family, prefix, cwd=tmp_path)
+    a, b = torch.load(os.path.join(theirs, "m.ref.logits")), torch.load(prefix + ".ours.logits")
     assert a.shape == b.shape and float((a - b).abs().max()) < 2e-6 * max(1.0, float(a.abs().max()))
 
 
@@ -644,13 +666,7 @@ def test_converted_checkpoint_scores_like_the_training_model_in_the_references_h
     import torch
     from safetensors.torch import load_file
 
-    ref, hf_code = _reference_root(), "/root/reference/transformers/internlm2_model"
-    if ref is None or not os.path.isdir(hf_code):
-        pytest.skip("the reference (and its transformers folder) is not available")
-    dst = str(tmp_path / "train_model.pt")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_model_probe.py"), ref, "INTERNLM2_PUBLIC", dst],
-                       capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-    assert r.returncode == 0 and "PROBE_OK" in r.stdout, r.stderr[-3000:]
+    dst = _model_probe("INTERNLM2_PUBLIC", tmp_path)
     probe = torch.load(dst, weights_only=False)
     ckpt = tmp_path / "ckpt"
     os.makedirs(ckpt)
@@ -665,13 +681,17 @@ def test_converted_checkpoint_scores_like_the_training_model_in_the_references_h
     for fn in os.listdir(tmp_path / "hf"):
         if fn.endswith(".safetensors"):
             weights.update(load_file(str(tmp_path / "hf" / fn)))
-    prefix = str(tmp_path / "conv")
-    torch.save(weights, prefix + ".hf_weights")
-    torch.save(probe["ids"], prefix + ".ids")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_hf_probe.py"), "load", hf_code, "internlm2", prefix],
-                       capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
-    assert r.returncode == 0 and "PROBE_OK" in r.stdout, r.stderr[-3000:]
-    hf_logits, train_logits = torch.load(prefix + ".load.logits"), probe["logits"]
+    def make(root, dst):
+        os.makedirs(dst, exist_ok=True)
+        torch.save(weights, os.path.join(dst, "conv.hf_weights"))
+        torch.save(probe["ids"], os.path.join(dst, "conv.ids"))
+        _probe("differential_hf_probe.py", "load", os.path.join(root, "transformers", "internlm2_model"), "internlm2",
+               os.path.join(dst, "conv"), cwd=tmp_path)
+
+    base = reference_output("converted_internlm2", make)
+    # the converter's output is what the reference's HF class was shown to load
+    assert_close(weights, torch.load(os.path.join(base, "conv.hf_weights")), "hf_weights")
+    hf_logits, train_logits = torch.load(os.path.join(base, "conv.load.logits")), probe["logits"]
     assert hf_logits.shape == train_logits.shape
     assert float((hf_logits - train_logits).abs().max()) < 2e-6 * max(1.0, float(train_logits.abs().max()))
 
@@ -682,16 +702,17 @@ def test_reverted_hf_model_scores_alike_in_the_references_training_model(tmp_pat
     import torch
     from safetensors.torch import save_file
 
-    ref, hf_code = _reference_root(), "/root/reference/transformers/internlm2_model"
-    if ref is None or not os.path.isdir(hf_code):
-        pytest.skip("the reference (and its transformers folder) is not available")
-    prefix, env = str(tmp_path / "hf"), dict(os.environ, CUDA_VISIBLE_DEVICES="", PROBE_INTERMEDIATE="256", PROBE_MLP_RATIO="8")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_hf_probe.py"), "ref", hf_code, "internlm2", prefix],
-                       capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=env)
-    assert r.returncode == 0 and "PROBE_OK" in r.stdout, r.stderr[-3000:]
+    env = dict(PROBE_INTERMEDIATE="256", PROBE_MLP_RATIO="8")
+
+    def make(root, dst):
+        os.makedirs(dst, exist_ok=True)
+        _probe("differential_hf_probe.py", "ref", os.path.join(root, "transformers", "internlm2_model"), "internlm2",
+               os.path.join(dst, "hf"), cwd=tmp_path, **env)
+
+    theirs = reference_output("hf_internlm2_mlp8", make)
     hf_dir = tmp_path / "hf_model"
     os.makedirs(hf_dir)
-    weights = {k: v.contiguous() for k, v in torch.load(prefix + ".weights").items() if "inv_freq" not in k}
+    weights = {k: v.contiguous() for k, v in torch.load(os.path.join(theirs, "hf.weights")).items() if "inv_freq" not in k}
     save_file(weights, str(hf_dir / "model.safetensors"))
     json.dump(dict(hidden_size=32, num_hidden_layers=2, num_attention_heads=4, num_key_value_heads=2, vocab_size=64,
                    intermediate_size=256, rms_norm_eps=1e-5, rope_theta=10000, bias=False, model_type="internlm2",
@@ -701,13 +722,19 @@ def test_reverted_hf_model_scores_alike_in_the_references_training_model(tmp_pat
     assert r.returncode == 0, r.stderr[-3000:]
     torch.manual_seed(1)
     ids = torch.randint(1, 64, (2, 12))          # the ids differential_hf_probe.py scored
-    given = str(tmp_path / "given.pt")
-    torch.save({"state": torch.load(tmp_path / "ckpt" / "model_tp0_pp0.pt", weights_only=False), "ids": ids}, given)
-    dst = str(tmp_path / "train_model.pt")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "differential_model_probe.py"), ref, "INTERNLM2_PUBLIC", dst, given],
-                       capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=env)
-    assert r.returncode == 0 and "PROBE_OK" in r.stdout, r.stderr[-3000:]
-    train_logits, hf_logits = torch.load(dst, weights_only=False)["logits"], torch.load(prefix + ".ref.logits")
+    state = torch.load(tmp_path / "ckpt" / "model_tp0_pp0.pt", weights_only=False)
+
+    def make_given(root, dst):
+        torch.save({"state": state, "ids": ids}, dst)
+
+    def make_logits(root, dst):
+        _probe("differential_model_probe.py", root, "INTERNLM2_PUBLIC", dst, given, cwd=tmp_path, **env)
+
+    given = reference_output("reverted_internlm2.pt", make_given)
+    # the reverted checkpoint is the one the reference's training model was shown to load
+    assert_close(state, torch.load(given, weights_only=False)["state"], "model_tp0_pp0.pt")
+    train_logits = torch.load(reference_output("reverted_internlm2.logits.pt", make_logits), weights_only=False)["logits"]
+    hf_logits = torch.load(os.path.join(theirs, "hf.ref.logits"))
     assert train_logits.shape == hf_logits.shape
     assert float((train_logits - hf_logits).abs().max()) < 2e-6 * max(1.0, float(hf_logits.abs().max()))
 
@@ -715,20 +742,22 @@ def test_reverted_hf_model_scores_alike_in_the_references_training_model(tmp_pat
 def test_alpaca_tokenizer_writes_the_references_bytes(tmp_path):
     """``tools/alpaca_tokenizer.py`` of both code bases on the same instruction data: chat template, negated prompt tokens, end-of-
     turn ids, truncation and the train / validation split give byte-identical ``dataset.bin`` files."""
-    ref_tool, model = "/root/reference/tools/alpaca_tokenizer.py", "/root/reference/tools/tokenizer_internlm.model"
-    if not (os.path.exists(ref_tool) and os.path.exists(model)):
-        pytest.skip("the reference's tools folder is not available")
+    model = _small_tokenizer_model(tmp_path)
     rng = np.random.RandomState(0)
     words = ["alpha", "beta", "gamma", "delta", "epsilon", "zeta", "数据", "模型"]
     data = [{"instruction": " ".join(rng.choice(words, 5)), "input": " ".join(rng.choice(words, 3)) if i % 2 else "",
              "output": " ".join(rng.choice(words, rng.randint(3, 2500 if i == 7 else 12)))} for i in range(60)]   # one over-long answer
     json.dump(data, open(tmp_path / "alpaca.json", "w"))
     env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
-    for tool, out, cwd in ((ref_tool, "ref", "/root/reference"), (os.path.join(ROOT, "tools", "alpaca_tokenizer.py"), "ours", str(tmp_path))):
-        r = subprocess.run([sys.executable, tool, str(tmp_path / "alpaca.json"), str(tmp_path / out), model, "--split_ratio", "0.1"],
-                           capture_output=True, text=True, timeout=600, cwd=cwd, env=env)
+
+    def run(tool, out):
+        r = subprocess.run([sys.executable, tool, str(tmp_path / "alpaca.json"), out, model, "--split_ratio", "0.1"],
+                           capture_output=True, text=True, timeout=600, cwd=str(tmp_path), env=env)
         assert r.returncode == 0, r.stderr[-2000:]
+
+    run(os.path.join(ROOT, "tools", "alpaca_tokenizer.py"), str(tmp_path / "ours"))
+    ref = reference_output("alpaca", lambda root, dst: run(os.path.join(root, "tools", "alpaca_tokenizer.py"), dst))
     for split in ("train", "valid"):
-        a = open(tmp_path / "ref" / split / "en" / "dataset.bin", "rb").read()
+        a = open(os.path.join(ref, split, "en", "dataset.bin"), "rb").read()
         b = open(tmp_path / "ours" / split / "en" / "dataset.bin", "rb").read()
         assert a == b and len(a) > 0, split
